@@ -144,8 +144,38 @@ def to_bf16(a):
     return (((u + 0x7FFF + ((u >> 16) & 1)) >> 16) & 0xFFFF).astype(np.uint16)
 
 
-def run_model(args, dist, rank, world, local_rank, dtype="f32", algorithm=-1, per_op_path=""):
-    """One measured configuration of the ResNet-50 step: returns the JSON object (rank 0 fills roofline / per_op)."""
+DUMP_SAMPLE = 1 << 21  # elements of each flat parameter / gradient buffer written by --dump-outputs (8 MB each in float32)
+
+
+def _as_float32(t):
+    """A tensor's contents as float32 (16-bit tensors are widened exactly)."""
+    a = t.download()
+    if a.dtype == np.uint16:  # bf16 bits
+        return (a.astype(np.uint32) << 16).view(np.float32)
+    return a.astype(np.float32)
+
+
+def dump_outputs(out_dir, net):
+    """What the last timed step handed back, as float32 .npy files: the per-sample loss, the logits and softmax probabilities
+    of its forward pass, and a fixed seeded sample (the same indices every run) of the parameters after its SGD update and of
+    the gradients its backward pass produced.  The model's inputs and initial weights are seeded, so two builds given the same
+    arguments can be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": _as_float32(net.loss), "logits": _as_float32(net.logits), "probs": _as_float32(net.probs)}
+    flats = [("params", net.w_flat), ("grads", net.g_flat)]
+    if hasattr(net, "w_flat_b"):  # 16-bit model: the fp32 batch-norm parameters and their gradients live in buffers of their own
+        flats += [("bn_params", net.w_flat_b), ("bn_grads", net.g_flat_b)]
+    for name, t in flats:
+        flat = _as_float32(t).reshape(-1)
+        idx = np.sort(np.random.RandomState(0).choice(flat.size, min(DUMP_SAMPLE, flat.size), replace=False))
+        arrays[name + "_sample"] = flat[idx]
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def run_model(args, dist, rank, world, local_rank, dtype="f32", algorithm=-1, per_op_path="", dump_dir=""):
+    """One measured configuration of the ResNet-50 step: returns the JSON object (rank 0 fills roofline / per_op).  dump_dir:
+    write the outputs of the last timed step there (dump_outputs)."""
     from ccv_b200 import nnc, resnet50
     device = local_rank
     dt = DTYPES[dtype]
@@ -240,6 +270,8 @@ def run_model(args, dist, rank, world, local_rank, dtype="f32", algorithm=-1, pe
     sampler.start()
     ms = timed(step, args.steps)
     ms_per_step = ms / args.steps
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, net)
 
     # end to end: every step copies its batch from pinned host memory and reads the loss back, through the same public calls
     # (CMD_DATA_TRANSFER on stream contexts).  The copy of batch k+1 runs on a second stream context while step k computes
@@ -303,11 +335,12 @@ def run_model(args, dist, rank, world, local_rank, dtype="f32", algorithm=-1, pe
     return out
 
 
-def run_sdpa_cfg5(args):
+def run_sdpa_cfg5(args, steps=None, warmup=3):
     """BASELINE.json configs[4]: CCV_NNC_SCALED_DOT_PRODUCT_ATTENTION_FORWARD bf16 B=32 H=16 S=2048 D=128, non-causal and causal,
     scale 1/sqrt(128), through ccv_nnc_cmd_exec; q / k / v are the reference's i / count ramps (test/int/nnc/cublas.tests.c:2786-2794)
     rounded to bf16.  Per variant: device-timed (CUDA events) with the operands resident in HBM, and end to end from pinned host
-    buffers (the three 268 MB operands in, the 268 MB result out, every step, inside the timed region)."""
+    buffers (the three 268 MB operands in, the 268 MB result out, every step, inside the timed region).  steps: timed steps of
+    every leg (None: 20 device-timed forwards, 5 end-to-end, 10 backwards, as measured next to the ResNet-50 step)."""
     from ccv_b200 import abi, nnc
     B, H, S, D = 32, 16, 2048, 128
     stream = nnc.Stream(0)
@@ -340,8 +373,8 @@ def run_sdpa_cfg5(args):
             fwd()
             nnc.cmd_exec(xfer, None, 0, [dev[3]], [host[3]], stream)
         res = {}
-        for name, fn, reps in (("device", fwd, 20), ("e2e", e2e, 5)):
-            for _ in range(3):
+        for name, fn, reps in (("device", fwd, steps or 20), ("e2e", e2e, steps or 5)):
+            for _ in range(warmup):
                 fn()
             e0, e1 = nnc.Event(), nnc.Event()
             stream.wait()
@@ -359,15 +392,15 @@ def run_sdpa_cfg5(args):
 
         def bwd():
             assert nnc.cmd_exec(bcmd, None, 0, b_ins, grads, stream) == 0, nnc.lib().ccv_nnc_sm100_last_error()
-        for _ in range(2):
+        for _ in range(warmup):
             bwd()
         e0, e1 = nnc.Event(), nnc.Event()
         stream.wait()
         e0.record(stream)
-        for _ in range(10):
+        for _ in range(steps or 10):
             bwd()
         e1.record(stream)
-        bms = e0.elapsed_ms(e1) / 10
+        bms = e0.elapsed_ms(e1) / (steps or 10)
         bflops = 10.0 * B * H * S * S * D * (0.5 if causal else 1.0)  # the 5 GEMMs of the backward; the kernels issue 7 (S and dP twice)
         flops = 4.0 * B * H * S * S * D * (0.5 if causal else 1.0)
         byts = 4.0 * n * 2 + B * H * S * 4
@@ -436,7 +469,10 @@ def main():
     ap.add_argument("--no-fuse", action="store_true", help="run every reference command as its own kernel sequence (no peephole fusion)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--per-op", default="", help="write the per-command profile to this JSON file")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR", help="write what the last timed step of the headline configuration computed to DIR/<name>.npy (float32, about 18 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.workload != "resnet50" or args.impl != "sm100"):
+        ap.error("--dump-outputs writes the outputs of the resnet50 workload on this backend only")
     if args.impl == "reference":
         return reference_arm(args)
     args.warmup = max(args.warmup, 3)
@@ -454,9 +490,9 @@ def main():
         raise SystemExit("bench.py: no CUDA device and there is no CPU fallback (use --impl reference for the CPU_REF arm)")
     if args.workload == "sdpa_cfg5":
         if rank == 0:
-            r = run_sdpa_cfg5(args)
+            r = run_sdpa_cfg5(args, args.steps, args.warmup)
             full = r["full"]
-            print(json.dumps({"metric": "sdpa_fwd_bf16_b32_h16_s2048_d128_tflops", "value": full["tflops"], "unit": "TFLOP/s", "n_gpus": 1, "steps": 20, "warmup": 3, "ms_per_step": full["ms"], "higher_is_better": True,
+            print(json.dumps({"metric": "sdpa_fwd_bf16_b32_h16_s2048_d128_tflops", "value": full["tflops"], "unit": "TFLOP/s", "n_gpus": 1, "steps": args.steps, "warmup": args.warmup, "ms_per_step": full["ms"], "higher_is_better": True,
                               "scaling": "weak", "vs_baseline": None, "dtype": "bf16", "data": "synthetic", "config": {"workload": r["workload"]},
                               "roofline": {"bound": "tensor", "achieved": full["tflops"], "peak": peaks()["bf16_tflops"], "unit": "TFLOP/s", "frac": full["frac_of_bf16_peak"], "traffic": None},
                               "e2e": {"value": full["e2e"]["tflops"], "unit": "TFLOP/s", "h2d_bytes_per_step": full["e2e"]["h2d_bytes_per_step"], "d2h_bytes_per_step": full["e2e"]["d2h_bytes_per_step"]},
@@ -466,7 +502,7 @@ def main():
             dist.destroy_process_group()
         return
 
-    out = run_model(args, dist, rank, world, local_rank, args.dtype, args.algorithm, args.per_op)
+    out = run_model(args, dist, rank, world, local_rank, args.dtype, args.algorithm, args.per_op, args.dump_outputs)
     if not args.no_variants:
         # the other BASELINE configurations, measured by the same code in the same process (same box, same clocks):
         #   bf16     configs[3] (ResNet-50 16-bit, batch-sharded): at N GPUs this IS configs[3]'s per-GPU shard of N x 256 images

@@ -54,7 +54,9 @@ def ref():
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     from oracle import ref as r
     if not r.available():
-        pytest.skip("oracle/_ref/libccv_ref.so not built (make -C oracle)")
+        # the outputs the compiled reference produced for these tests, stored under tests/golden/cpu_ref (tests/util.py)
+        from tests.util import StoredRef
+        return StoredRef()
     r.ref()
     # the parity cases are small: a handful of OpenMP threads serves them better than one per hardware thread of a large host (the GPU
     # suite spent most of its time in oversubscribed CPU_REF parallel regions); results do not depend on the count

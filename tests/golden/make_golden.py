@@ -1,14 +1,22 @@
 """Regenerates tests/golden/*.npz from the reference's own known-answer tests and from the compiled reference
-(oracle/_ref/libccv_ref.so).  Run in the build container (needs /root/reference built through `make -C oracle`):
+(oracle/_ref/libccv_ref.so).  Run where the reference sources are present and `make -C oracle` has built the compiled reference:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py          # everything below
+    python tests/golden/make_golden.py facts    # reference_facts.json only
 
-Two kinds of fixtures:
+The CPU_REF outputs of the parity tests (tests/golden/cpu_ref/) are written by the tests themselves: run the suite on a GPU
+machine with CCV_REF_RECORD=1 and the compiled reference present (tests/util.py).
+
+Three kinds of fixtures here:
   literal_*   inputs + expected outputs typed from the reference's unit tests (test/unit/nnc/gemm.tests.c etc.); these
               pin the oracle itself.
   cpuref_*    seeded inputs + the outputs CCV_NNC_BACKEND_CPU_REF produced for them here; these travel to the GPU box
               so parity can be checked even without the compiled reference.
+  reference_facts.json   the reference's struct layouts, ccv_nnc_hint_auto results and the digest of its float -> half bit patterns
+                         (tests/test_abi.py, tests/test_oracle.py).
 """
+import hashlib
+import json
 import os
 import sys
 
@@ -66,8 +74,38 @@ def cpuref_cases():
     return cases
 
 
+def reference_facts():
+    """What the compiled reference reports about itself: its struct sizes / field offsets (ref_shim.c:ref_abi_sizes) and the hints
+    ccv_nnc_hint_auto derives for tests/test_oracle.py HINT_AUTO_CASES (raw ccv_nnc_hint_t bytes, hex)."""
+    import ctypes as C
+    from ccv_b200 import abi
+    from tests.test_oracle import HINT_AUTO_CASES
+    sizes = (C.c_int * 10)()
+    ref.ref().ref_abi_sizes(sizes)
+    hints = []
+    for case in HINT_AUTO_CASES:
+        size, a_dims, b_dims = case[:3]
+        kind = case[3] if len(case) > 3 else "nhwc"
+        fa = abi.CCV_TENSOR_FORMAT_NHWC if kind in ("nhwc", "mixed") else abi.CCV_TENSOR_FORMAT_NCHW
+        fb = abi.CCV_TENSOR_FORMAT_NHWC if kind == "nhwc" else abi.CCV_TENSOR_FORMAT_NCHW
+        info = abi.CmdParam()
+        for j, d in enumerate(size):
+            info.size.dim[j] = d
+        pa = abi.tensor_param(abi.CCV_TENSOR_CPU_MEMORY, fa, abi.CCV_32F, list(a_dims), 0)
+        pb = abi.tensor_param(abi.CCV_TENSOR_CPU_MEMORY, fb, abi.CCV_32F, list(b_dims), 0)
+        h = abi.Hint()
+        ref.ref().ref_hint_auto(C.byref(info), C.byref(pa), C.byref(pb), C.byref(h))
+        hints.append(bytes(h).hex())
+    from tests.test_oracle import F2H_INPUT
+    return dict(abi_sizes=list(sizes), hint_auto=hints, float_to_half_sha256=hashlib.sha256(ref.float_to_half(F2H_INPUT()).tobytes()).hexdigest())
+
+
 if __name__ == "__main__":
+    if sys.argv[1:] == ["facts"]:  # only reference_facts.json
+        json.dump(reference_facts(), open(os.path.join(OUT, "reference_facts.json"), "w"), indent=1)
+        sys.exit(0)
     np.savez(os.path.join(OUT, "literal_gemm.npz"), **literal_gemm())
     for name, d in cpuref_cases().items():
         np.savez(os.path.join(OUT, "cpuref_%s.npz" % name), **d)
+    json.dump(reference_facts(), open(os.path.join(OUT, "reference_facts.json"), "w"), indent=1)
     print("wrote", sorted(os.listdir(OUT)))

@@ -3,6 +3,8 @@ and tensor identities, so its rewrites can be checked without a device (nothing 
 Rewrite (f) (convolution -> batch-norm statistics) needs a device allocation and is covered by the GPU tests."""
 import ctypes as C
 
+import pytest
+
 from ccv_b200 import abi, nnc
 
 

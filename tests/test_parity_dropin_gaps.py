@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 
 from ccv_b200 import abi
-from tests.util import NCHW, NHWC, assert_close, gpu_exec, gpu_exec16, ref_exec, round16, seeded
+from tests.util import NCHW, NHWC, assert_close, gpu_exec, gpu_exec16, max_abs_diff, ref_exec, round16, same, seeded
 
 pytestmark = [pytest.mark.gpu, pytest.mark.ref]
 
@@ -90,7 +90,7 @@ def test_fp32_only_commands_on_16bit_tensors(gpu, ref, kind):
         assert st == 0, name
         assert_close(o_g, o_r, 1e-2, name)
     g = round16(seeded((10, 100), 3, -1, 1), kind)
-    _, (p_r,) = ref_exec(ref, nnc.CMD_SOFTMAX_FORWARD(), None, 0, [x], [z()])
+    _, (p_r,) = ref_exec(ref, nnc.CMD_SOFTMAX_FORWARD(), None, 0, [x], [z()], whole=True)  # the backward's operand is made from it
     p16 = round16(p_r, kind)
     _, (h_r,) = ref_exec(ref, nnc.CMD_SOFTMAX_BACKWARD(), None, 0, [g, None, p16], [z()])
     st, (h_g,) = gpu_exec16(nnc, nnc.CMD_SOFTMAX_BACKWARD(), None, 0, [g, None, p16], [z()], kind)
@@ -122,11 +122,11 @@ def test_pooling_nchw(gpu, ref, which):
         xc = np.ascontiguousarray(x.transpose(perm))
         st, (y_g,) = gpu_exec(nnc, fwd(k, k), hint, 0, [xc], [np.zeros(tuple(np.array(out_nhwc)[list(perm)]), np.float32)], fmt=NCHW)
         assert st == 0
-        assert np.array_equal(y_g.transpose(back), y_r) if which == "max" else np.abs(y_g.transpose(back) - y_r).max() <= 1e-6
+        assert same(y_g.transpose(back), y_r) if which == "max" else max_abs_diff(y_g.transpose(back), y_r) <= 1e-6
         g = seeded(out_nhwc, 2, -1, 1)
         ins_r = [g, x, y_r] if which == "max" else [g]
         _, (h_r,) = ref_exec(ref, bwd(k, k), hint, 0, ins_r, [np.zeros(shape_nhwc, np.float32)])
-        gc, yc = np.ascontiguousarray(g.transpose(perm)), np.ascontiguousarray(y_r.transpose(perm))
+        gc, yc = np.ascontiguousarray(g.transpose(perm)), y_g  # each side's backward reads its own forward output (compared above)
         ins_g = [gc, xc, yc] if which == "max" else [gc]
         st, (h_g,) = gpu_exec(nnc, bwd(k, k), hint, 0, ins_g, [np.zeros(xc.shape, np.float32)], fmt=NCHW)
         assert st == 0

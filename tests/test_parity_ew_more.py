@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 
 from ccv_b200 import abi
-from tests.util import assert_close, gpu_exec, gpu_exec16, ref_exec, round16, seeded
+from tests.util import assert_close, gpu_exec, gpu_exec16, max_abs, max_abs_diff, ref_exec, round16, same, seeded
 
 pytestmark = [pytest.mark.gpu, pytest.mark.ref]
 NAN = float("nan")
@@ -18,6 +18,10 @@ def _z(shape=SHAPE):
     return np.zeros(shape, np.float32)
 
 
+NUMPY = {  # the forward in float64, for an operand both sides are given
+    "SIGMOID": lambda x: 1 / (1 + np.exp(-x)), "TANH": np.tanh, "LEAKY_RELU": lambda x: np.where(x > 0, x, 0.2 * x), "EWEXP": np.exp,
+    "EWLOG": np.log, "EWSQRT": np.sqrt, "CLAMP": lambda x: np.clip(x, -0.5, 0.75),
+}
 UNARY = {
     # name: (forward ctor args, input range, which operand the backward reads: 1 = a, 2 = b)
     "SIGMOID": ((), (-6, 6), 2), "TANH": ((), (-3, 3), 2), "LEAKY_RELU": ((0.2,), (-2, 2), 2), "EWEXP": ((), (-3, 3), 2),
@@ -36,20 +40,19 @@ def test_unary_forward_backward(gpu, ref, name):
     assert st == 0
     exact = name in ("CLAMP", "LEAKY_RELU")
     if exact:
-        assert np.array_equal(y_g, y_r), name
+        assert same(y_g, y_r), name
     else:
         assert_close(y_g, y_r, 1e-5, name + " forward")
-    ins = [g, x, y_r] if which == 2 else [g, x]
-    _, (h_r,) = ref_exec(ref, bwd, None, 0, ins, [_z()])
-    st, (h_g,) = gpu_exec(nnc, bwd, None, 0, ins, [_z()])
+    # each side's backward reads its own forward output (compared above)
+    _, (h_r,) = ref_exec(ref, bwd, None, 0, [g, x, y_r] if which == 2 else [g, x], [_z()])
+    st, (h_g,) = gpu_exec(nnc, bwd, None, 0, [g, x, y_g] if which == 2 else [g, x], [_z()])
     assert st == 0
     assert_close(h_g, h_r, 1e-5, name + " backward")
     if name == "EWEXP":
         # no incoming gradient = all ones (ew_cpu_ref.c:1043-1044; CPU_REF's sigmoid / tanh backward dereference g before testing it,
         # sigmoid_cpu_ref.c:44, so that form has no oracle there)
-        ins0 = [None, x, y_r]
-        _, (h0_r,) = ref_exec(ref, bwd, None, 0, ins0, [_z()])
-        st, (h0_g,) = gpu_exec(nnc, bwd, None, 0, ins0, [_z()])
+        _, (h0_r,) = ref_exec(ref, bwd, None, 0, [None, x, y_r], [_z()])
+        st, (h0_g,) = gpu_exec(nnc, bwd, None, 0, [None, x, y_g], [_z()])
         assert st == 0
         assert_close(h0_g, h0_r, 1e-5, name + " backward without g")
     # bf16: oracle on rounded inputs
@@ -58,7 +61,7 @@ def test_unary_forward_backward(gpu, ref, name):
     st, (yb_g,) = gpu_exec16(nnc, fwd, None, 0, [xb], [_z()], abi.CCV_16BF)
     assert st == 0
     assert_close(yb_g, yb_r, 1e-2, name + " forward bf16")
-    yb = round16(yb_r, abi.CCV_16BF)
+    yb = round16(NUMPY[name](xb.astype(np.float64)).astype(np.float32), abi.CCV_16BF)  # the bf16 forward output, as an operand
     insb = [gb, xb, yb] if which == 2 else [gb, xb]
     _, (hb_r,) = ref_exec(ref, bwd, None, 0, insb, [_z()])
     st, (hb_g,) = gpu_exec16(nnc, bwd, None, 0, insb, [_z()], abi.CCV_16BF)
@@ -72,11 +75,11 @@ def test_clamp_open_sides(gpu, ref):
     for lo, hi in ((NAN, 0.5), (-0.25, NAN)):
         _, (y_r,) = ref_exec(ref, nnc.CMD_CLAMP_FORWARD(lo, hi), None, 0, [x], [_z()])
         st, (y_g,) = gpu_exec(nnc, nnc.CMD_CLAMP_FORWARD(lo, hi), None, 0, [x], [_z()])
-        assert st == 0 and np.array_equal(y_g, y_r)
+        assert st == 0 and same(y_g, y_r)
         g = seeded(SHAPE, 4, -1, 1)
         _, (h_r,) = ref_exec(ref, nnc.CMD_CLAMP_BACKWARD(lo, hi), None, 0, [g, x, y_r], [_z()])
         st, (h_g,) = gpu_exec(nnc, nnc.CMD_CLAMP_BACKWARD(lo, hi), None, 0, [g, x, y_r], [_z()])
-        assert st == 0 and np.array_equal(h_g, h_r)
+        assert st == 0 and same(h_g, h_r)
 
 
 def test_ewdiv_forward_backward(gpu, ref):
@@ -91,7 +94,7 @@ def test_ewdiv_forward_backward(gpu, ref):
     assert st == 0
     assert_close(r_g, r_r, 1e-6, "1 / b")
     _, (ha_r, hb_r) = ref_exec(ref, nnc.CMD_EWDIV_BACKWARD(), None, 0, [g, a, b, c_r], [_z(), _z()])
-    st, (ha_g, hb_g) = gpu_exec(nnc, nnc.CMD_EWDIV_BACKWARD(), None, 0, [g, a, b, c_r], [_z(), _z()])
+    st, (ha_g, hb_g) = gpu_exec(nnc, nnc.CMD_EWDIV_BACKWARD(), None, 0, [g, a, b, c_g], [_z(), _z()])  # each side's own quotient
     assert st == 0
     assert_close(ha_g, ha_r, 1e-5, "d(a / b) / da")
     assert_close(hb_g, hb_r, 1e-5, "d(a / b) / db")
@@ -115,14 +118,13 @@ def test_reduce_forward_backward(gpu, ref, mode, shape, axes):
     st, (y_g,) = gpu_exec(nnc, fwd, None, 0, [x], [_z(out_shape)])
     assert st == 0
     if mode in ("MAX", "MIN"):
-        assert np.array_equal(y_g, y_r), mode
+        assert same(y_g, y_r), mode
     else:
         # the bound is relative to the magnitude of what is summed, not of a sum that may cancel
-        err = np.abs(y_g - y_r).max() / max(np.abs(x).sum(axis=axes).max() * (1.0 / np.prod([shape[a] for a in axes]) if mode == "MEAN" else 1.0), 1e-30)
-        assert err <= 1e-5 if mode != "NORM2" else np.abs(y_g - y_r).max() <= 1e-5 * np.abs(y_r).max(), (mode, err)
-    ins = [g, x, y_r]
-    _, (h_r,) = ref_exec(ref, bwd, None, 0, ins, [_z(shape)])
-    st, (h_g,) = gpu_exec(nnc, bwd, None, 0, ins, [_z(shape)])
+        err = max_abs_diff(y_g, y_r) / max(np.abs(x).sum(axis=axes).max() * (1.0 / np.prod([shape[a] for a in axes]) if mode == "MEAN" else 1.0), 1e-30)
+        assert err <= 1e-5 if mode != "NORM2" else max_abs_diff(y_g, y_r) <= 1e-5 * max_abs(y_r), (mode, err)
+    _, (h_r,) = ref_exec(ref, bwd, None, 0, [g, x, y_r], [_z(shape)])
+    st, (h_g,) = gpu_exec(nnc, bwd, None, 0, [g, x, y_g], [_z(shape)])  # each side's own forward output (compared above)
     assert st == 0
     assert_close(h_g, h_r, 1e-6, "reduce %s backward" % mode)
     if mode in ("SUM", "MEAN"):
@@ -153,11 +155,11 @@ def test_masked_fill(gpu, ref, mask_dtype):
     fwd, bwd = nnc.CMD_MASKED_FILL_FORWARD(2, -1e9), nnc.CMD_MASKED_FILL_BACKWARD(2, -1e9)
     _, (c_r,) = ref_exec(ref, fwd, None, 0, [a, mask], [_z(shape)])
     st, (c_g,) = gpu_exec(nnc, fwd, None, 0, [a, mask], [_z(shape)])
-    assert st == 0 and np.array_equal(c_g, c_r)
+    assert st == 0 and same(c_g, c_r)
     assert (c_g == -1e9).sum() == (np.broadcast_to(mask, shape) == 2).sum()
     _, (h_r,) = ref_exec(ref, bwd, None, 0, [g, None, mask], [_z(shape)])
     st, (h_g,) = gpu_exec(nnc, bwd, None, 0, [g, None, mask], [_z(shape)])
-    assert st == 0 and np.array_equal(h_g, h_r)
+    assert st == 0 and same(h_g, h_r)
 
 
 @pytest.mark.parametrize("n", [100003, 4096])

@@ -91,7 +91,8 @@ def test_group_norm_forward_backward(gpu, ref, shape, group_axis, groups, reduce
         ins = [g, None, None, x, None, m_r, s_r]
         mk = lambda: [np.zeros(shape, np.float32)]
     st_r, outs_r = ref_exec(ref, bwd, None, 0, ins, mk())
-    st_g, outs_g = gpu_exec(nnc, bwd, None, 0, ins, mk())
+    ins_g = [m_g if a is m_r else s_g if a is s_r else a for a in ins]  # each side's own saved statistics (compared above)
+    st_g, outs_g = gpu_exec(nnc, bwd, None, 0, ins_g, mk())
     assert st_r == 0 and st_g == 0
     for name, a, b in zip(("dx", "dscale", "dbias"), outs_g, outs_r):
         assert_close(a, b, 1e-3, name)

@@ -12,6 +12,8 @@ the TEACHER-FORCED test: every one of the ~550 forward + backward nodes is execu
 values the oracle saw in front of that node, and its outputs are compared with the oracle's outputs of the same node
 (fp32 FFMA <= 1e-3, one-pass TF32 <= 1e-2 normalised max error; bit-for-bit ops are not separated out here).
 Also: the fused graph (peephole pass) and its CUDA-graph replay must reproduce the unfused eager result."""
+import os
+
 import numpy as np
 import pytest
 
@@ -40,8 +42,46 @@ def _gpu_net(nnc, algo, fuse, stream):
     return net, g, fused
 
 
+STORED = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "cpu_ref", "resnet50_cpu_net.npz")
+GRAD_SAMPLE = 1 << 12  # stored elements of the flat gradient (seeded positions)
+
+
+def _grad_positions(n):
+    return np.sort(np.random.RandomState(11).choice(n, min(GRAD_SAMPLE, n), replace=False))
+
+
+class _Stored(object):
+    """What the CPU_REF run of the model produced, as stored by a recording run (CCV_REF_RECORD=1): logits, probabilities and
+    loss whole, the flat gradient at _grad_positions.  No per-node snapshots."""
+
+    class _T(object):
+        def __init__(self, a):
+            self.a = a
+
+        def download(self):
+            return self.a.copy()
+
+    def __init__(self, path):
+        z = np.load(path)
+        self.logits, self.probs, self.loss = self._T(z["logits"]), self._T(z["probs"]), self._T(z["loss"])
+        self.grad_sample, self.grad_count = z["grad_sample"], int(z["grad_count"])
+
+
+def _grads(net, cpu_net):
+    """(this backend's flat gradient, CPU_REF's) as float64: whole, or at the stored positions."""
+    gg = net.g_flat.download().astype(np.float64)
+    if isinstance(cpu_net, _Stored):
+        assert gg.size == cpu_net.grad_count
+        return gg[_grad_positions(gg.size)], cpu_net.grad_sample.astype(np.float64)
+    return gg, cpu_net.g_flat.download().astype(np.float64)
+
+
 @pytest.fixture(scope="module")
 def cpu_net(ref):
+    if getattr(ref, "stored", False):
+        if not os.path.exists(STORED):
+            pytest.skip("no stored CPU_REF run of the model (%s) and the compiled reference is not built" % os.path.relpath(STORED))
+        return _Stored(STORED)
     from oracle import ref_factory
     x, lab = _inputs()
     cpu = resnet50.Net(BATCH, image=IMAGE, classes=CLASSES, factory=ref_factory.RefFactory(), seed=7)
@@ -56,6 +96,11 @@ def cpu_net(ref):
         cpu.snap_out.append([None if t is None else t.download() for t in node[4]])
 
     ref_factory.run_nodes(cpu.fwd + cpu.bwd, before, after)
+    if os.environ.get("CCV_REF_RECORD"):
+        g = cpu.g_flat.download()
+        os.makedirs(os.path.dirname(STORED), exist_ok=True)
+        np.savez_compressed(STORED, logits=cpu.logits.download(), probs=cpu.probs.download(), loss=cpu.loss.download(),
+                            grad_sample=g[_grad_positions(g.size)], grad_count=np.array(g.size))
     return cpu
 
 
@@ -68,7 +113,7 @@ def test_resnet50_forward_backward_vs_cpu_ref(gpu, cpu_net, algo, tol_out, tol_g
     assert_close(net.logits.download(), cpu_net.logits.download(), tol_out, "logits")
     assert_close(net.probs.download(), cpu_net.probs.download(), tol_out, "softmax")
     assert_close(net.loss.download(), cpu_net.loss.download(), tol_out, "loss")
-    gg, gc = net.g_flat.download().astype(np.float64), cpu_net.g_flat.download().astype(np.float64)
+    gg, gc = _grads(net, cpu_net)
     assert np.isfinite(gg).all()
     rel_l2 = np.linalg.norm(gg - gc) / np.linalg.norm(gc)
     cos = float(gg @ gc / (np.linalg.norm(gg) * np.linalg.norm(gc)))
@@ -80,6 +125,8 @@ def test_resnet50_forward_backward_vs_cpu_ref(gpu, cpu_net, algo, tol_out, tol_g
 @pytest.mark.ref
 @pytest.mark.parametrize("algo,tol", [(abi.CCV_NNC_SM100_ALGO_FFMA, 1e-3), (abi.CCV_NNC_SM100_ALGO_3XTF32, 1e-3), (abi.CCV_NNC_SM100_ALGO_TF32, 1e-2)])
 def test_resnet50_every_node_teacher_forced_vs_cpu_ref(gpu, cpu_net, algo, tol):
+    if isinstance(cpu_net, _Stored):
+        pytest.skip("feeds every node the compiled reference's own operands (oracle/_ref/libccv_ref.so, make -C oracle): too large to store")
     nnc = gpu
     stream = nnc.Stream(0)
     net = resnet50.Net(BATCH, image=IMAGE, classes=CLASSES, seed=7, algorithm=algo)
@@ -168,7 +215,7 @@ def test_fused_cuda_graph_vs_cpu_ref(gpu, cpu_net, algo, tol):
     assert_close(net.logits.download(), cpu_net.logits.download(), tol, "logits (fused, CUDA graph)")
     assert_close(net.probs.download(), cpu_net.probs.download(), tol, "softmax (fused, CUDA graph)")
     assert_close(net.loss.download(), cpu_net.loss.download(), tol, "loss (fused, CUDA graph)")
-    gg, gc = net.g_flat.download().astype(np.float64), cpu_net.g_flat.download().astype(np.float64)
+    gg, gc = _grads(net, cpu_net)
     assert np.isfinite(gg).all()
     cos = float(gg @ gc / (np.linalg.norm(gg) * np.linalg.norm(gc)))
     print("algo %d fused + captured: gradient cosine vs CPU_REF %.6f" % (algo, cos))
