@@ -772,12 +772,14 @@ int ccv_nnc_sm100_fused_sgd_multi(const ccv_nnc_cmd_t, const ccv_nnc_hint_t, con
 int ccv_nnc_sm100_fused_conv_stats_forw(const ccv_nnc_cmd_t, const ccv_nnc_hint_t, const int, ccv_nnc_tensor_t* const*, const int, ccv_nnc_tensor_t* const*, const int, ccv_nnc_stream_context_t*);
 int ccv_nnc_sm100_fused_bn_forw(const ccv_nnc_cmd_t, const ccv_nnc_hint_t, const int, ccv_nnc_tensor_t* const*, const int, ccv_nnc_tensor_t* const*, const int, ccv_nnc_stream_context_t*);
 int ccv_nnc_sm100_fused_bn_back(const ccv_nnc_cmd_t, const ccv_nnc_hint_t, const int, ccv_nnc_tensor_t* const*, const int, ccv_nnc_tensor_t* const*, const int, ccv_nnc_stream_context_t*);
+int ccv_nnc_sm100_fused_bn_add_relu_forw(const ccv_nnc_cmd_t, const ccv_nnc_hint_t, const int, ccv_nnc_tensor_t* const*, const int, ccv_nnc_tensor_t* const*, const int, ccv_nnc_stream_context_t*);
+int ccv_nnc_sm100_fused_add_relu_back_stats(const ccv_nnc_cmd_t, const ccv_nnc_hint_t, const int, ccv_nnc_tensor_t* const*, const int, ccv_nnc_tensor_t* const*, const int, ccv_nnc_stream_context_t*);
 }
 
 struct ccv_nnc_sm100_graph_s {
 	std::vector<ccv_nnc_sm100_graph_node_t> nodes;
 	std::vector<cudaGraphExec_t> captures;
-	std::vector<ccv_nnc_tensor_t*> owned; // statistics tensors of fused convolution -> batch-norm pairs
+	std::vector<ccv_nnc_tensor_t*> owned; // small tensors the fusion rewrites pass between the two nodes of a pair (statistics, coefficients)
 	// second stream context for nodes marked `side` (gradient-exchange commands that overlap the rest of the backward pass), on the
 	// device of the stream the graph runs on; two reusable signals order it with the main stream (what the reference's graph
 	// runner does with per-node wait / emit signals across its streams, lib/nnc/ccv_nnc_graph_run.c:451-543)
@@ -921,6 +923,7 @@ int ccv_nnc_sm100_graph_run(ccv_nnc_sm100_graph_t* const graph, const int begin,
 //  (d) EWSUM(a, b -> a) ; RELU_BACKWARD in place on a (mask y)                -> a = y > 0 ? a + b : 0
 //  (e) a run of SGD_FORWARD nodes with identical parameters (the per-parameter updates of a model; none of them reads
 //      what another one writes) -> one multi-tensor command; counts as (run length - 1) fused nodes
+// (f) - (i) below pair nodes without removing either.
 int ccv_nnc_sm100_graph_fuse(ccv_nnc_sm100_graph_t* const graph)
 {
 	std::vector<ccv_nnc_sm100_graph_node_t>& nodes = graph->nodes;
@@ -1091,6 +1094,110 @@ int ccv_nnc_sm100_graph_fuse(ccv_nnc_sm100_graph_t* const graph)
 			if (!b.fused)
 				b.fused = ccv_nnc_sm100_fused_bn_back;
 		}
+	// The end of a residual block: the last batch norm of the main branch (no ReLU), the shortcut add and the ReLU.
+	// CCV_NNC_SM100_FUSE_BLOCK_END=0 turns (h) and (i) off.  Neither removes a node.
+	const char* const env_end = getenv("CCV_NNC_SM100_FUSE_BLOCK_END");
+	const bool block_end = !env_end || atoi(env_end) != 0;
+	auto same_mem = [](const ccv_nnc_tensor_t* const x, const ccv_nnc_tensor_t* const y) { return x == y || (x && y && x->data.u8 && x->data.u8 == y->data.u8); };
+	auto plain_node = [](const ccv_nnc_sm100_graph_node_t& x) { return !x.side && (x.cmd.backend == CCV_NNC_BACKEND_GPU_SM100 || x.cmd.backend == CCV_NNC_NO_BACKEND); };
+	// the batch norm normalises the innermost dimension of a packed GPU tensor (NHWC): C of it, or 0
+	auto nhwc_channels = [](const ccv_nnc_tensor_t* const x, const ccv_nnc_tensor_t* const scale) {
+		if (!x || !scale || CCV_IS_TENSOR_VIEW(x) || CCV_IS_TENSOR_VIEW(scale) || CCV_TENSOR_GET_MEMORY(x->info.type) != CCV_TENSOR_GPU_MEMORY)
+			return 0;
+		int nd = 0;
+		size_t count = 1;
+		while (nd < CCV_NNC_MAX_DIM_ALLOC && scale->info.dim[nd] > 0)
+			count *= (size_t)scale->info.dim[nd++];
+		if (nd == 0 || (size_t)scale->info.dim[nd - 1] != count)
+			return 0;
+		int xnd = 0;
+		while (xnd < CCV_NNC_MAX_DIM_ALLOC && x->info.dim[xnd] > 0)
+			xnd++;
+		return xnd > 0 && x->info.dim[xnd - 1] == (int)count ? (int)count : 0;
+	};
+	auto owned_f32 = [&](const ccv_nnc_tensor_t* const like, const int rows, const int cols) -> ccv_nnc_tensor_t* {
+		ccv_nnc_tensor_param_t params = like->info;
+		memset(params.dim, 0, sizeof(params.dim));
+		params.dim[0] = rows, params.dim[1] = cols;
+		params.datatype = CCV_32F;
+		ccv_nnc_tensor_t* const t = ccv_nnc_tensor_new(0, params, 0);
+		if (!t || !t->data.u8)
+		{
+			if (t)
+				ccv_nnc_tensor_free(t);
+			return 0;
+		}
+		t->sig = 0;
+		graph->owned.push_back(t);
+		return t;
+	};
+	// (h) BATCH_NORM_FORWARD(train, no ReLU; plain or reading convolution statistics) ; the fused add + ReLU (c) whose first operand
+	//     is the batch norm's output y, which no later node reads: the batch norm only computes the statistics and leaves its
+	//     per-channel a, b in a [2, C] tensor owned by the graph; the add node computes relu(x * a + b + shortcut) from the batch
+	//     norm's input x.  y is never written (one write and one read of the activation fewer).
+	if (block_end)
+		for (size_t i = 0; i + 1 < out.size(); i++)
+		{
+			ccv_nnc_sm100_graph_node_t& b = out[i];
+			ccv_nnc_sm100_graph_node_t& e = out[i + 1];
+			if (!plain_node(b) || b.cmd.cmd != CCV_NNC_BATCH_NORM_FORWARD || b.cmd.info.bnorm.is_test || (b.fused && b.fused != ccv_nnc_sm100_fused_bn_forw) || (b.inputs.size() != 5 && b.inputs.size() != 6) || b.outputs.size() != 5 || !b.outputs[0])
+				continue;
+			if (!plain_node(e) || e.fused != ccv_nnc_sm100_fused_add_relu_forw || e.inputs.size() != 2 || e.inputs[0] != b.outputs[0] || same_mem(e.inputs[1], b.outputs[0]) || same_mem(e.outputs[0], b.outputs[0]))
+				continue;
+			const int C = nhwc_channels(b.inputs[0], b.inputs[1]);
+			if (!C)
+				continue;
+			bool y_read_later = false;
+			for (size_t j = i + 2; j < out.size() && !y_read_later; j++)
+				for (ccv_nnc_tensor_t* t : out[j].inputs)
+					if (same_mem(t, b.outputs[0]))
+					{
+						y_read_later = true;
+						break;
+					}
+			if (y_read_later)
+				continue;
+			ccv_nnc_tensor_t* const coef = owned_f32(b.inputs[1], 2, C);
+			if (!coef)
+				continue;
+			b.outputs.push_back(coef);
+			if (!b.fused)
+				b.fused = ccv_nnc_sm100_fused_bn_forw;
+			e.inputs[0] = b.inputs[0];
+			e.inputs.push_back(coef);
+			e.fused = ccv_nnc_sm100_fused_bn_add_relu_forw;
+		}
+	// (i) the fused add + ReLU backward (d), or a RELU_BACKWARD left plain by (b) ; BATCH_NORM_BACKWARD (no ReLU; plain or with the
+	//     convolution's bias gradient of (g)) of its output: the first node also produces the batch norm's reduction over (g, x)
+	//     as per-block partial rows in a tensor owned by the graph; the batch norm only finalises and applies (one read of g fewer).
+	if (block_end)
+		for (size_t i = 0; i + 1 < out.size(); i++)
+		{
+			ccv_nnc_sm100_graph_node_t& r = out[i];
+			ccv_nnc_sm100_graph_node_t& b = out[i + 1];
+			if (!plain_node(r) || r.inputs.size() != 3 || r.outputs.size() != 1 || !r.inputs[0] || !r.inputs[2] || !r.outputs[0])
+				continue;
+			if (!(r.fused == ccv_nnc_sm100_fused_add_relu_back || (!r.fused && r.cmd.cmd == CCV_NNC_RELU_BACKWARD)))
+				continue;
+			if (!plain_node(b) || b.cmd.cmd != CCV_NNC_BATCH_NORM_BACKWARD || (b.fused && b.fused != ccv_nnc_sm100_fused_bn_back) || b.inputs.size() != 15 || b.inputs[0] != r.outputs[0] || b.inputs[7] || !b.inputs[5] || !b.inputs[13])
+				continue;
+			const int C = nhwc_channels(b.inputs[5], b.inputs[6]);
+			if (!C)
+				continue;
+			// room for bn_reduce_kernel's grid rows: at most 4 per SM (reduce_config), for up to 160 SMs
+			ccv_nnc_tensor_t* const part = owned_f32(b.inputs[13], 4 * 160 + 8, 2 * C);
+			if (!part)
+				continue;
+			if (!r.fused) // RELU_BACKWARD (g, -, y): the add's second operand stays empty
+				r.inputs[1] = 0;
+			r.inputs.push_back(b.inputs[5]);
+			r.inputs.push_back(b.inputs[13]);
+			r.outputs.push_back(part);
+			r.fused = ccv_nnc_sm100_fused_add_relu_back_stats;
+			b.inputs.push_back(part);
+			if (!b.fused)
+				b.fused = ccv_nnc_sm100_fused_bn_back;
+		}
 	nodes.swap(out);
 	return fused;
 }
@@ -1102,7 +1209,7 @@ int ccv_nnc_sm100_graph_node(const ccv_nnc_sm100_graph_t* const graph, const int
 		return -1;
 	const ccv_nnc_sm100_graph_node_t& n = graph->nodes[i];
 	*cmd = n.cmd.cmd;
-	*fused_kind = n.fused == ccv_nnc_sm100_fused_bn_relu_forw ? 1 : n.fused == ccv_nnc_sm100_fused_relu_bn_back ? 2 : n.fused == ccv_nnc_sm100_fused_add_relu_forw ? 3 : n.fused == ccv_nnc_sm100_fused_add_relu_back ? 4 : n.fused == ccv_nnc_sm100_fused_sgd_multi ? 5 : n.fused == ccv_nnc_sm100_fused_conv_stats_forw ? 6 : n.fused == ccv_nnc_sm100_fused_bn_forw ? 7 : n.fused == ccv_nnc_sm100_fused_bn_back ? 8 : 0;
+	*fused_kind = n.fused == ccv_nnc_sm100_fused_bn_relu_forw ? 1 : n.fused == ccv_nnc_sm100_fused_relu_bn_back ? 2 : n.fused == ccv_nnc_sm100_fused_add_relu_forw || n.fused == ccv_nnc_sm100_fused_bn_add_relu_forw ? 3 : n.fused == ccv_nnc_sm100_fused_add_relu_back || n.fused == ccv_nnc_sm100_fused_add_relu_back_stats ? 4 : n.fused == ccv_nnc_sm100_fused_sgd_multi ? 5 : n.fused == ccv_nnc_sm100_fused_conv_stats_forw ? 6 : n.fused == ccv_nnc_sm100_fused_bn_forw ? 7 : n.fused == ccv_nnc_sm100_fused_bn_back ? 8 : 0;
 	*input_size = (int)n.inputs.size();
 	*output_size = (int)n.outputs.size();
 	return 0;

@@ -1125,7 +1125,12 @@ int bnorm_forw(const int fuse_relu, const ccv_nnc_cmd_t cmd, const ccv_nnc_hint_
 			RC(bn_fwd_test_16(s, kind, inputs[0]->data.u8, outputs[0]->data.u8, inputs[1]->data.f32, inputs[2]->data.f32, inputs[3]->data.f32, inputs[4]->data.f32, outer, C, inner, cmd.info.bnorm.epsilon, tws));
 		return CCV_NNC_EXEC_SUCCESS;
 	}
-	if (output_size != 5 || !outputs[1] || !outputs[2] || !outputs[3] || !outputs[4])
+	// a 6th output is the [2, C] fp32 coefficient tensor of a statistics-only batch norm (rewrite (h) of ccv_nnc_sm100_graph_fuse):
+	// it receives the a, b of y = x * a + b and y itself is not written -- the residual add behind it applies them
+	ccv_nnc_tensor_t* const coef_t = output_size == 6 ? outputs[5] : 0;
+	if ((output_size != 5 && !coef_t) || !outputs[1] || !outputs[2] || !outputs[3] || !outputs[4])
+		return CCV_NNC_EXEC_INVALID;
+	if (coef_t && (fuse_relu || !is_f32(coef_t) || !view_of(coef_t).contiguous || view_of(coef_t).count != 2 * (size_t)C))
 		return CCV_NNC_EXEC_INVALID;
 	// running mean / var are updated in place (:45-46)
 	if (inputs[3]->data.f32 != outputs[1]->data.f32 || inputs[4]->data.f32 != outputs[2]->data.f32)
@@ -1140,10 +1145,10 @@ int bnorm_forw(const int fuse_relu, const ccv_nnc_cmd_t cmd, const ccv_nnc_hint_
 			return CCV_NNC_EXEC_INVALID;
 	if (kind == 0)
 		RC(bn_fwd_train_f32(s, inputs[0]->data.f32, outputs[0]->data.f32, inputs[1]->data.f32, inputs[2]->data.f32, outputs[1]->data.f32, outputs[2]->data.f32, outputs[3]->data.f32, outputs[4]->data.f32, outer, C, inner, cmd.info.bnorm.epsilon, cmd.info.bnorm.momentum, ws, fuse_relu,
-			stats_t && inner == 1 ? stats_t->data.f32 : 0, stats_t ? (int)stats_t->sig : 0));
+			stats_t && inner == 1 ? stats_t->data.f32 : 0, stats_t ? (int)stats_t->sig : 0, coef_t ? coef_t->data.f32 : 0));
 	else
 		RC(bn_fwd_train_16(s, kind, inputs[0]->data.u8, outputs[0]->data.u8, inputs[1]->data.f32, inputs[2]->data.f32, outputs[1]->data.f32, outputs[2]->data.f32, outputs[3]->data.f32, outputs[4]->data.f32, outer, C, inner, cmd.info.bnorm.epsilon, cmd.info.bnorm.momentum, ws, fuse_relu,
-			stats_t && inner == 1 ? stats_t->data.f32 : 0, stats_t ? (int)stats_t->sig : 0));
+			stats_t && inner == 1 ? stats_t->data.f32 : 0, stats_t ? (int)stats_t->sig : 0, coef_t ? coef_t->data.f32 : 0));
 	return CCV_NNC_EXEC_SUCCESS;
 }
 
@@ -1158,8 +1163,11 @@ static inline bool h_t_ok(const ccv_nnc_tensor_t* const h) { return h != 0; }
 // outputs (h, dscale, dbias)
 int bnorm_back(const int fused_relu, const ccv_nnc_cmd_t cmd, const ccv_nnc_hint_t hint, const int flags, ccv_nnc_tensor_t* const* const inputs, const int input_size, ccv_nnc_tensor_t* const* const outputs, const int output_size, ccv_nnc_stream_context_t* const stream_context)
 {
-	if (input_size != 15 || output_size < 1)
+	if ((input_size != 15 && input_size != 16) || output_size < 1)
 		return CCV_NNC_EXEC_INVALID;
+	// a 16th input is the partial-row tensor the add + ReLU backward in front filled (rewrite (i) of ccv_nnc_sm100_graph_fuse): its
+	// `sig` field carries the number of rows written for this issue (0 = none: reduce here)
+	const ccv_nnc_tensor_t* const part_t = input_size == 16 ? inputs[15] : 0;
 	// the fused form carries the forward bias in slot 7 (unused by BATCH_NORM_BACKWARD, norm/ccv_nnc_norm.c:28-37)
 	const ccv_nnc_tensor_t* const bias_t = fused_relu ? inputs[7] : 0;
 	if (fused_relu && !bias_t)
@@ -1189,15 +1197,18 @@ int bnorm_back(const int fused_relu, const ccv_nnc_cmd_t cmd, const ccv_nnc_hint
 		return CCV_NNC_EXEC_INVALID;
 	if (h_t && (!same_shape(view_of(h_t), a) || !view_of(h_t).contiguous))
 		return CCV_NNC_EXEC_INVALID;
+	const bool ext = part_t && !fused_relu && inner == 1 && part_t->sig > 0 && is_f32(part_t) && part_t->info.dim[1] == 2 * C && (int)part_t->sig <= part_t->info.dim[0];
+	const float* const ext_part = ext ? part_t->data.f32 : 0;
+	const int ext_rows = ext ? (int)part_t->sig : 0;
 	cudaStream_t s = stream_of(stream_context);
 	void* const ws = ccv_nnc_stream_context_get_workspace(stream_context, bn_workspace_bytes(C), CCV_TENSOR_GPU_MEMORY);
 	if (!ws)
 		return CCV_NNC_EXEC_OOM;
 	if (kind == 0 && (!conv_dbias_t || is_f32(conv_dbias_t)))
-		RC(bn_bwd_f32(s, g_t->data.f32, a_t->data.f32, scale_t->data.f32, bias_t ? bias_t->data.f32 : 0, mean_t->data.f32, istd_t->data.f32, h_t ? h_t->data.f32 : 0, dscale_t ? dscale_t->data.f32 : 0, dbias_t ? dbias_t->data.f32 : 0, outer, C, inner, ws, conv_dbias_t ? conv_dbias_t->data.f32 : 0));
+		RC(bn_bwd_f32(s, g_t->data.f32, a_t->data.f32, scale_t->data.f32, bias_t ? bias_t->data.f32 : 0, mean_t->data.f32, istd_t->data.f32, h_t ? h_t->data.f32 : 0, dscale_t ? dscale_t->data.f32 : 0, dbias_t ? dbias_t->data.f32 : 0, outer, C, inner, ws, conv_dbias_t ? conv_dbias_t->data.f32 : 0, ext_part, ext_rows));
 	else if (kind != 0)
 		RC(bn_bwd_16(s, kind, g_t->data.u8, a_t->data.u8, scale_t->data.f32, bias_t ? bias_t->data.f32 : 0, mean_t->data.f32, istd_t->data.f32, h_t ? (void*)h_t->data.u8 : 0, dscale_t ? dscale_t->data.f32 : 0, dbias_t ? dbias_t->data.f32 : 0, outer, C, inner, ws,
-			conv_dbias_t ? (void*)conv_dbias_t->data.u8 : 0, conv_dbias_t ? kind_of(conv_dbias_t) : 0));
+			conv_dbias_t ? (void*)conv_dbias_t->data.u8 : 0, conv_dbias_t ? kind_of(conv_dbias_t) : 0, ext_part, ext_rows));
 	else
 		return CCV_NNC_EXEC_INVALID;
 	return CCV_NNC_EXEC_SUCCESS;
@@ -2240,6 +2251,57 @@ extern "C" int ccv_nnc_sm100_fused_add_relu_back(const ccv_nnc_cmd_t cmd, const 
 		RC(ew_add_relu_bwd_16(stream_of(stream_context), kind, inputs[0]->data.u8, inputs[1]->data.u8, inputs[2]->data.u8, outputs[0]->data.u8, o.count));
 	else
 		RC(ew_add_relu_bwd_f32(stream_of(stream_context), inputs[0]->data.f32, inputs[1]->data.f32, inputs[2]->data.f32, outputs[0]->data.f32, o.count));
+	return CCV_NNC_EXEC_SUCCESS;
+}
+
+// The end of a residual block with the batch norm of the main branch folded in (rewrite (h)): inputs (x, shortcut, coef) ->
+// out = relu(x * a + b + shortcut), where coef ([2, C] fp32) holds the a, b a statistics-only BATCH_NORM_FORWARD just wrote.
+// NHWC: the channel is the innermost dimension.  Bit-identical to BATCH_NORM_FORWARD, EWSUM, RELU_FORWARD.
+extern "C" int ccv_nnc_sm100_fused_bn_add_relu_forw(const ccv_nnc_cmd_t cmd, const ccv_nnc_hint_t hint, const int flags, ccv_nnc_tensor_t* const* const inputs, const int input_size, ccv_nnc_tensor_t* const* const outputs, const int output_size, ccv_nnc_stream_context_t* const stream_context)
+{
+	if (input_size != 3 || output_size != 1 || !inputs[0] || !inputs[1] || !inputs[2] || !outputs[0])
+		return CCV_NNC_EXEC_INVALID;
+	const TV x = view_of(inputs[0]), r = view_of(inputs[1]), c = view_of(inputs[2]), y = view_of(outputs[0]);
+	const int kind = kind_of(outputs[0]);
+	if (!x.contiguous || !r.contiguous || !y.contiguous || !c.contiguous || !is_f32(inputs[2]) || x.count != y.count || r.count != y.count || kind < 0 || kind_of(inputs[0]) != kind || kind_of(inputs[1]) != kind || x.nd < 1)
+		return CCV_NNC_EXEC_INVALID;
+	const int C = x.dim[x.nd - 1];
+	if (C <= 0 || c.count != 2 * (size_t)C)
+		return CCV_NNC_EXEC_INVALID;
+	if (kind != 0)
+		RC(bn_add_relu_fwd_16(stream_of(stream_context), kind, inputs[0]->data.u8, inputs[1]->data.u8, outputs[0]->data.u8, inputs[2]->data.f32, x.count / C, C));
+	else
+		RC(bn_add_relu_fwd_f32(stream_of(stream_context), inputs[0]->data.f32, inputs[1]->data.f32, outputs[0]->data.f32, inputs[2]->data.f32, x.count / C, C));
+	return CCV_NNC_EXEC_SUCCESS;
+}
+
+// The add + ReLU backward of a residual block end (b = NULL: a plain RELU_BACKWARD) carrying the reduction of the batch-norm
+// backward behind it (rewrite (i)): inputs (a, b, y, x, saved_mean) -> outputs (g, part); g = y > 0 ? a + b : 0 and part
+// ([rows, 2C] fp32) receives the per-block partial sums of g and g * (x - mean), their number in its `sig` field (0 when the layout
+// takes the plain path; the batch norm then reduces g itself).  x / mean are that batch norm's input and saved mean, NHWC.
+extern "C" int ccv_nnc_sm100_fused_add_relu_back_stats(const ccv_nnc_cmd_t cmd, const ccv_nnc_hint_t hint, const int flags, ccv_nnc_tensor_t* const* const inputs, const int input_size, ccv_nnc_tensor_t* const* const outputs, const int output_size, ccv_nnc_stream_context_t* const stream_context)
+{
+	if (input_size != 5 || output_size != 2 || !inputs[0] || !inputs[2] || !inputs[3] || !inputs[4] || !outputs[0] || !outputs[1])
+		return CCV_NNC_EXEC_INVALID;
+	ccv_nnc_tensor_t* const part_t = outputs[1];
+	part_t->sig = 0;
+	const TV a = view_of(inputs[0]), y = view_of(inputs[2]), x = view_of(inputs[3]), m = view_of(inputs[4]), o = view_of(outputs[0]);
+	const int kind = kind_of(outputs[0]);
+	if (!a.contiguous || !y.contiguous || !x.contiguous || !o.contiguous || a.count != o.count || y.count != o.count || x.count != o.count || kind < 0 || kind_of(inputs[0]) != kind || kind_of(inputs[2]) != kind || kind_of(inputs[3]) != kind)
+		return CCV_NNC_EXEC_INVALID;
+	if (inputs[1] && (!view_of(inputs[1]).contiguous || view_of(inputs[1]).count != o.count || kind_of(inputs[1]) != kind))
+		return CCV_NNC_EXEC_INVALID;
+	if (!is_f32(inputs[4]) || !is_f32(part_t) || x.nd < 1)
+		return CCV_NNC_EXEC_INVALID;
+	// the reduction is only done for the batch norm's NHWC layout: one statistic per innermost element, a [rows, 2C] partial tensor
+	const int C = x.dim[x.nd - 1];
+	const int cap = C > 0 && m.count == (size_t)C && part_t->info.dim[1] == 2 * C ? part_t->info.dim[0] : 0;
+	int rows = 0;
+	if (kind != 0)
+		RC(bn_add_relu_bwd_reduce_16(stream_of(stream_context), kind, inputs[0]->data.u8, inputs[1] ? inputs[1]->data.u8 : 0, inputs[2]->data.u8, inputs[3]->data.u8, inputs[4]->data.f32, outputs[0]->data.u8, o.count / (cap ? C : 1), cap ? C : 1, cap ? part_t->data.f32 : 0, cap, &rows));
+	else
+		RC(bn_add_relu_bwd_reduce_f32(stream_of(stream_context), inputs[0]->data.f32, inputs[1] ? inputs[1]->data.f32 : 0, inputs[2]->data.f32, inputs[3]->data.f32, inputs[4]->data.f32, outputs[0]->data.f32, o.count / (cap ? C : 1), cap ? C : 1, cap ? part_t->data.f32 : 0, cap, &rows));
+	part_t->sig = (uint64_t)rows;
 	return CCV_NNC_EXEC_SUCCESS;
 }
 

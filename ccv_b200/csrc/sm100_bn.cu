@@ -58,8 +58,12 @@ static inline float* ws_part(void* ws, int C) { return (float*)(((uintptr_t)(ws_
 // NHWC: thread = (column-vector tx, row-lane ty); each thread walks rows with 4 independent 128-bit loads in flight.
 // MODE 0: s1 = sum(x - k), s2 = sum((x - k)^2), k = x[0, c] (shift keeps the one-pass variance well conditioned).
 // MODE 1: s1 = sum(g'), s2 = sum(g' * (x - mean)); g' = g, or g masked by relu(x * a + b) > 0 when MASK.
+// MODE 2: MODE 1 on g' = ym > 0 ? ga + gb : 0 (gb may be NULL: ym > 0 ? ga : 0), which is also stored to gout -- the residual
+//         block end's add + ReLU backward feeding the batch-norm reduction behind it.  The row walk and the in-block combine are
+//         those of MODE 1, so the partial rows are bit-identical to storing g' first and reducing it with MODE 1.
 template <typename T, int MODE, int MASK>
-__global__ void __launch_bounds__(256) bn_reduce_kernel(const T* __restrict__ x, const T* __restrict__ g, const float* __restrict__ mean, const float* __restrict__ coef, const size_t rows, const int C, float* __restrict__ part, const int cpb)
+__global__ void __launch_bounds__(256) bn_reduce_kernel(const T* __restrict__ x, const T* __restrict__ g, const float* __restrict__ mean, const float* __restrict__ coef, const size_t rows, const int C, float* __restrict__ part, const int cpb,
+	const T* __restrict__ ga = 0, const T* __restrict__ gb = 0, const T* __restrict__ ym = 0, T* __restrict__ gout = 0)
 {
 	// one 16-byte access = W channels (4 fp32 / 8 bf16 or fp16); thread = (channel group tx, row lane ty)
 	constexpr int W = Vec16<T>::W;
@@ -102,6 +106,17 @@ __global__ void __launch_bounds__(256) bn_reduce_kernel(const T* __restrict__ x,
 				}
 			}
 		};
+		// MODE 2: g' of one row from the two branch gradients and the block output, rounded to T as a store would round it
+		auto grad = [&](const size_t off, float (&gv)[W]) {
+			float u[W], v[W], m[W];
+			ldv(ga + off, u), ldv(ym + off, m);
+			if (gb)
+				ldv(gb + off, v);
+#pragma unroll
+			for (int k = 0; k < W; k++)
+				gv[k] = rnd<T>(m[k] > 0.f ? (gb ? u[k] + v[k] : u[k]) : 0.f);
+			stv(gout + off, gv);
+		};
 		for (; r + 3 * step < rows; r += 4 * step)
 		{
 			float xv[4][W], gv[4][W];
@@ -111,10 +126,12 @@ __global__ void __launch_bounds__(256) bn_reduce_kernel(const T* __restrict__ x,
 				ldv(x + (r + u * step) * C + cw * W, xv[u]);
 				if (MODE == 1)
 					ldv(g + (r + u * step) * C + cw * W, gv[u]);
+				else if (MODE == 2)
+					grad((r + u * step) * C + cw * W, gv[u]);
 			}
 #pragma unroll
 			for (int u = 0; u < 4; u++)
-				acc(xv[u], MODE == 1 ? gv[u] : xv[u]);
+				acc(xv[u], MODE >= 1 ? gv[u] : xv[u]);
 		}
 		for (; r < rows; r += step)
 		{
@@ -122,7 +139,9 @@ __global__ void __launch_bounds__(256) bn_reduce_kernel(const T* __restrict__ x,
 			ldv(x + r * C + cw * W, xv);
 			if (MODE == 1)
 				ldv(g + r * C + cw * W, gv);
-			acc(xv, MODE == 1 ? gv : xv);
+			else if (MODE == 2)
+				grad(r * C + cw * W, gv);
+			acc(xv, MODE >= 1 ? gv : xv);
 		}
 	}
 #pragma unroll
@@ -492,7 +511,9 @@ __global__ void __launch_bounds__(256) bn_apply_vec_kernel(const T* __restrict__
 // into registers instead of on every iteration (they were 4 of the 6 loads per element group: the pass was L1 / issue bound at
 // 0.5 of the HBM rate, worse for 16-bit data), every access is 16 bytes (4 fp32 or 8 bf16 / fp16 elements) and four row loads
 // are in flight per thread.  COLSUM as above.
-template <typename T, int BWD, int RELU, int COLSUM>
+// RES (forward, no RELU): g is a residual operand and out = relu(roundT(x * a + b) + g) -- the batch norm at the end of a residual
+// block, the shortcut add and the ReLU in one pass, rounded as the batch norm's own store would round before the add.
+template <typename T, int BWD, int RELU, int COLSUM, int RES = 0>
 __global__ void __launch_bounds__(256) bn_apply_fixed_kernel(const T* __restrict__ x, const T* __restrict__ g, T* __restrict__ out, const float* __restrict__ coef, const size_t totalw, const int C, float* __restrict__ part)
 {
 	constexpr int W = Vec16<T>::W;
@@ -516,7 +537,7 @@ __global__ void __launch_bounds__(256) bn_apply_fixed_kernel(const T* __restrict
 			if (i + u * stride < totalw)
 			{
 				ldv(x + (i + u * stride) * W, xv[u]);
-				if (BWD)
+				if (BWD || RES)
 					ldv(g + (i + u * stride) * W, gv[u]);
 			}
 #pragma unroll
@@ -527,7 +548,9 @@ __global__ void __launch_bounds__(256) bn_apply_fixed_kernel(const T* __restrict
 #pragma unroll
 				for (int k = 0; k < W; k++)
 				{
-					if (!BWD)
+					if (RES)
+						o[k] = fmaxf(rnd<T>(fmaf(xv[u][k], a[k], b[k])) + gv[u][k], 0.f);
+					else if (!BWD)
 					{
 						o[k] = fmaf(xv[u][k], a[k], b[k]);
 						if (RELU)
@@ -597,14 +620,16 @@ __global__ void __launch_bounds__(1024) bn_colsum_rows_kernel(const float* __res
 		st_kind(out, c, t, out_kind);
 	}
 }
-template <typename T, int BWD, int RELU>
+template <typename T, int BWD, int RELU, int RES = 0>
 __global__ void bn_apply_generic_kernel(const T* __restrict__ x, const T* __restrict__ g, T* __restrict__ out, const float* __restrict__ coef, const size_t total, const int C, const size_t inner)
 {
 	for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x)
 	{
 		const int c = (int)((i / inner) % C);
 		const float a = coef[c], b = coef[C + c], xv = ldf(x + i);
-		if (!BWD)
+		if (RES)
+			stf(out + i, fmaxf(rnd<T>(fmaf(xv, a, b)) + ldf(g + i), 0.f));
+		else if (!BWD)
 		{
 			const float o = fmaf(xv, a, b);
 			stf(out + i, RELU ? fmaxf(o, 0.f) : o);
@@ -700,12 +725,13 @@ static int run_apply(cudaStream_t s, const T* x, const T* g, T* out, const float
 }
 
 template <typename T>
-static int bn_fwd_train_t(cudaStream_t s, const T* x, T* y, const float* scale, const float* bias, float* running_mean, float* running_var, float* saved_mean, float* saved_inv_std, size_t outer, int C, size_t inner, float epsilon, float momentum, void* workspace, int fuse_relu, const float* ext_part, int ext_rows)
+static int bn_fwd_train_t(cudaStream_t s, const T* x, T* y, const float* scale, const float* bias, float* running_mean, float* running_var, float* saved_mean, float* saved_inv_std, size_t outer, int C, size_t inner, float epsilon, float momentum, void* workspace, int fuse_relu, const float* ext_part, int ext_rows, float* coef_out)
 {
 	if (outer * C * inner == 0)
 		return 0;
 	double* ws = ws_sums(workspace);
-	float* coef = ws_coef(workspace, C);
+	// coef_out: statistics only -- the per-channel a, b go to the caller's [2, C] buffer and y is not written
+	float* coef = coef_out ? coef_out : ws_coef(workspace, C);
 	int part_rows = 0;
 	if (ext_part && ext_rows > 0)
 	{
@@ -713,6 +739,8 @@ static int bn_fwd_train_t(cudaStream_t s, const T* x, T* y, const float* scale, 
 		bn_finalize_ext_kernel<<<(C + 31) / 32, 1024, 0, s>>>(ext_part, ext_rows, C, epsilon, momentum, scale, bias, running_mean, running_var, saved_mean, saved_inv_std, coef);
 		if (check("bn_fwd_finalize(ext)"))
 			return -1;
+		if (coef_out)
+			return 0;
 		return fuse_relu ? run_apply<T, 0, 1>(s, x, (const T*)0, y, coef, outer, C, inner) : run_apply<T, 0, 0>(s, x, (const T*)0, y, coef, outer, C, inner);
 	}
 	if (run_reduce<T, 0, 0>(s, x, (const T*)0, 0, 0, outer, C, inner, ws, ws_part(workspace, C), &part_rows))
@@ -723,6 +751,8 @@ static int bn_fwd_train_t(cudaStream_t s, const T* x, T* y, const float* scale, 
 		bn_fwd_finalize_kernel<T><<<(C + 127) / 128, 128, 0, s>>>(x, inner, ws, C, (double)outer * (double)inner, epsilon, momentum, scale, bias, running_mean, running_var, saved_mean, saved_inv_std, coef);
 	if (check("bn_fwd_finalize"))
 		return -1;
+	if (coef_out)
+		return 0;
 	return fuse_relu ? run_apply<T, 0, 1>(s, x, (const T*)0, y, coef, outer, C, inner) : run_apply<T, 0, 0>(s, x, (const T*)0, y, coef, outer, C, inner);
 }
 
@@ -739,8 +769,9 @@ static int bn_fwd_test_t(cudaStream_t s, const T* x, T* y, const float* scale, c
 }
 
 // bias != NULL selects the fused form: g is the gradient w.r.t. relu(bn(x)) and is masked by bn(x) > 0 on the fly
+// ext_part / ext_rows: the partial rows of the reduction over (g, x), already produced by bn_add_relu_bwd_reduce_t
 template <typename T>
-static int bn_bwd_t(cudaStream_t s, const T* g, const T* x, const float* scale, const float* bias, const float* saved_mean, const float* saved_inv_std, T* dx, float* dscale, float* dbias, size_t outer, int C, size_t inner, void* workspace, void* dx_colsum, int colsum_kind)
+static int bn_bwd_t(cudaStream_t s, const T* g, const T* x, const float* scale, const float* bias, const float* saved_mean, const float* saved_inv_std, T* dx, float* dscale, float* dbias, size_t outer, int C, size_t inner, void* workspace, void* dx_colsum, int colsum_kind, const float* ext_part, int ext_rows)
 {
 	if (outer * C * inner == 0)
 		return 0;
@@ -760,13 +791,16 @@ static int bn_bwd_t(cudaStream_t s, const T* g, const T* x, const float* scale, 
 			return -1;
 	}
 	int part_rows = 0;
-	if (mask ? run_reduce<T, 1, 1>(s, x, g, saved_mean, coef, outer, C, inner, ws, ws_part(workspace, C), &part_rows) : run_reduce<T, 1, 0>(s, x, g, saved_mean, coef, outer, C, inner, ws, ws_part(workspace, C), &part_rows))
+	const float* part_in = ws_part(workspace, C);
+	if (ext_part && ext_rows > 0 && vec && !mask)
+		part_in = ext_part, part_rows = ext_rows;
+	else if (mask ? run_reduce<T, 1, 1>(s, x, g, saved_mean, coef, outer, C, inner, ws, ws_part(workspace, C), &part_rows) : run_reduce<T, 1, 0>(s, x, g, saved_mean, coef, outer, C, inner, ws, ws_part(workspace, C), &part_rows))
 		return -1;
 	const double count = (double)outer * (double)inner;
 	if (part_rows > 0 && mask)
-		bn_finalize_partials_kernel<T, 1, 0><<<(C + 31) / 32, 1024, 0, s>>>(ws_part(workspace, C), part_rows, (const T*)0, C, count, 0.f, 0.f, scale, 0, 0, 0, const_cast<float*>(saved_mean), const_cast<float*>(saved_inv_std), dscale, dbias, coef);
+		bn_finalize_partials_kernel<T, 1, 0><<<(C + 31) / 32, 1024, 0, s>>>(part_in, part_rows, (const T*)0, C, count, 0.f, 0.f, scale, 0, 0, 0, const_cast<float*>(saved_mean), const_cast<float*>(saved_inv_std), dscale, dbias, coef);
 	else if (part_rows > 0)
-		bn_finalize_partials_kernel<T, 1, 1><<<(C + 31) / 32, 1024, 0, s>>>(ws_part(workspace, C), part_rows, (const T*)0, C, count, 0.f, 0.f, scale, 0, 0, 0, const_cast<float*>(saved_mean), const_cast<float*>(saved_inv_std), dscale, dbias, coef);
+		bn_finalize_partials_kernel<T, 1, 1><<<(C + 31) / 32, 1024, 0, s>>>(part_in, part_rows, (const T*)0, C, count, 0.f, 0.f, scale, 0, 0, 0, const_cast<float*>(saved_mean), const_cast<float*>(saved_inv_std), dscale, dbias, coef);
 	else
 		bn_bwd_finalize_kernel<<<(C + 127) / 128, 128, 0, s>>>(ws, C, (float)count, scale, saved_mean, saved_inv_std, dscale, dbias, coef);
 	if (check("bn_bwd_finalize"))
@@ -784,25 +818,25 @@ static int bn_bwd_t(cudaStream_t s, const T* g, const T* x, const float* scale, 
 	return 0;
 }
 
-int bn_fwd_train_f32(cudaStream_t s, const float* x, float* y, const float* scale, const float* bias, float* running_mean, float* running_var, float* saved_mean, float* saved_inv_std, size_t outer, int C, size_t inner, float epsilon, float momentum, void* workspace, int fuse_relu, const float* ext_part, int ext_rows)
+int bn_fwd_train_f32(cudaStream_t s, const float* x, float* y, const float* scale, const float* bias, float* running_mean, float* running_var, float* saved_mean, float* saved_inv_std, size_t outer, int C, size_t inner, float epsilon, float momentum, void* workspace, int fuse_relu, const float* ext_part, int ext_rows, float* coef_out)
 {
-	return bn_fwd_train_t<float>(s, x, y, scale, bias, running_mean, running_var, saved_mean, saved_inv_std, outer, C, inner, epsilon, momentum, workspace, fuse_relu, ext_part, ext_rows);
+	return bn_fwd_train_t<float>(s, x, y, scale, bias, running_mean, running_var, saved_mean, saved_inv_std, outer, C, inner, epsilon, momentum, workspace, fuse_relu, ext_part, ext_rows, coef_out);
 }
 int bn_fwd_test_f32(cudaStream_t s, const float* x, float* y, const float* scale, const float* bias, const float* mean, const float* var, size_t outer, int C, size_t inner, float epsilon, void* workspace)
 {
 	return bn_fwd_test_t<float>(s, x, y, scale, bias, mean, var, outer, C, inner, epsilon, workspace);
 }
-int bn_bwd_f32(cudaStream_t s, const float* g, const float* x, const float* scale, const float* bias, const float* saved_mean, const float* saved_inv_std, float* dx, float* dscale, float* dbias, size_t outer, int C, size_t inner, void* workspace, float* dx_colsum)
+int bn_bwd_f32(cudaStream_t s, const float* g, const float* x, const float* scale, const float* bias, const float* saved_mean, const float* saved_inv_std, float* dx, float* dscale, float* dbias, size_t outer, int C, size_t inner, void* workspace, float* dx_colsum, const float* ext_part, int ext_rows)
 {
-	return bn_bwd_t<float>(s, g, x, scale, bias, saved_mean, saved_inv_std, dx, dscale, dbias, outer, C, inner, workspace, dx_colsum, 0);
+	return bn_bwd_t<float>(s, g, x, scale, bias, saved_mean, saved_inv_std, dx, dscale, dbias, outer, C, inner, workspace, dx_colsum, 0, ext_part, ext_rows);
 }
 // 16-bit activations (kind 1 = bf16, 2 = fp16); scale / bias / statistics / parameter gradients stay fp32
 // (lib/nnc/ccv_cnnp_model_addons.c:954-956)
-int bn_fwd_train_16(cudaStream_t s, int kind, const void* x, void* y, const float* scale, const float* bias, float* running_mean, float* running_var, float* saved_mean, float* saved_inv_std, size_t outer, int C, size_t inner, float epsilon, float momentum, void* workspace, int fuse_relu, const float* ext_part, int ext_rows)
+int bn_fwd_train_16(cudaStream_t s, int kind, const void* x, void* y, const float* scale, const float* bias, float* running_mean, float* running_var, float* saved_mean, float* saved_inv_std, size_t outer, int C, size_t inner, float epsilon, float momentum, void* workspace, int fuse_relu, const float* ext_part, int ext_rows, float* coef_out)
 {
 	if (kind == 1)
-		return bn_fwd_train_t<__nv_bfloat16>(s, (const __nv_bfloat16*)x, (__nv_bfloat16*)y, scale, bias, running_mean, running_var, saved_mean, saved_inv_std, outer, C, inner, epsilon, momentum, workspace, fuse_relu, ext_part, ext_rows);
-	return bn_fwd_train_t<__half>(s, (const __half*)x, (__half*)y, scale, bias, running_mean, running_var, saved_mean, saved_inv_std, outer, C, inner, epsilon, momentum, workspace, fuse_relu, ext_part, ext_rows);
+		return bn_fwd_train_t<__nv_bfloat16>(s, (const __nv_bfloat16*)x, (__nv_bfloat16*)y, scale, bias, running_mean, running_var, saved_mean, saved_inv_std, outer, C, inner, epsilon, momentum, workspace, fuse_relu, ext_part, ext_rows, coef_out);
+	return bn_fwd_train_t<__half>(s, (const __half*)x, (__half*)y, scale, bias, running_mean, running_var, saved_mean, saved_inv_std, outer, C, inner, epsilon, momentum, workspace, fuse_relu, ext_part, ext_rows, coef_out);
 }
 int bn_fwd_test_16(cudaStream_t s, int kind, const void* x, void* y, const float* scale, const float* bias, const float* mean, const float* var, size_t outer, int C, size_t inner, float epsilon, void* workspace)
 {
@@ -810,11 +844,11 @@ int bn_fwd_test_16(cudaStream_t s, int kind, const void* x, void* y, const float
 		return bn_fwd_test_t<__nv_bfloat16>(s, (const __nv_bfloat16*)x, (__nv_bfloat16*)y, scale, bias, mean, var, outer, C, inner, epsilon, workspace);
 	return bn_fwd_test_t<__half>(s, (const __half*)x, (__half*)y, scale, bias, mean, var, outer, C, inner, epsilon, workspace);
 }
-int bn_bwd_16(cudaStream_t s, int kind, const void* g, const void* x, const float* scale, const float* bias, const float* saved_mean, const float* saved_inv_std, void* dx, float* dscale, float* dbias, size_t outer, int C, size_t inner, void* workspace, void* dx_colsum, int colsum_kind)
+int bn_bwd_16(cudaStream_t s, int kind, const void* g, const void* x, const float* scale, const float* bias, const float* saved_mean, const float* saved_inv_std, void* dx, float* dscale, float* dbias, size_t outer, int C, size_t inner, void* workspace, void* dx_colsum, int colsum_kind, const float* ext_part, int ext_rows)
 {
 	if (kind == 1)
-		return bn_bwd_t<__nv_bfloat16>(s, (const __nv_bfloat16*)g, (const __nv_bfloat16*)x, scale, bias, saved_mean, saved_inv_std, (__nv_bfloat16*)dx, dscale, dbias, outer, C, inner, workspace, dx_colsum, colsum_kind);
-	return bn_bwd_t<__half>(s, (const __half*)g, (const __half*)x, scale, bias, saved_mean, saved_inv_std, (__half*)dx, dscale, dbias, outer, C, inner, workspace, dx_colsum, colsum_kind);
+		return bn_bwd_t<__nv_bfloat16>(s, (const __nv_bfloat16*)g, (const __nv_bfloat16*)x, scale, bias, saved_mean, saved_inv_std, (__nv_bfloat16*)dx, dscale, dbias, outer, C, inner, workspace, dx_colsum, colsum_kind, ext_part, ext_rows);
+	return bn_bwd_t<__half>(s, (const __half*)g, (const __half*)x, scale, bias, saved_mean, saved_inv_std, (__half*)dx, dscale, dbias, outer, C, inner, workspace, dx_colsum, colsum_kind, ext_part, ext_rows);
 }
 
 // ------------------------------------------------------------------------------------------------ fused residual adds
@@ -872,6 +906,76 @@ int ew_add_relu_fwd_16(cudaStream_t s, int kind, const void* a, const void* b, v
 int ew_add_relu_bwd_16(cudaStream_t s, int kind, const void* a, const void* b, const void* y, void* out, size_t n)
 {
 	return kind == 1 ? add_relu_bwd_t<__nv_bfloat16>(s, (const __nv_bfloat16*)a, (const __nv_bfloat16*)b, (const __nv_bfloat16*)y, (__nv_bfloat16*)out, n) : add_relu_bwd_t<__half>(s, (const __half*)a, (const __half*)b, (const __half*)y, (__half*)out, n);
+}
+
+// ------------------------------------------------------------------------------------------------ residual block end
+// Forward: out = relu(roundT(x * a + b) + r) with the [2, C] coefficients a statistics-only batch norm left in coef (NHWC, C =
+// the innermost dimension); the same bits as the batch-norm apply pass followed by add_relu_kernel, without writing / reading
+// the normalised tensor in between.
+template <typename T>
+static int bn_add_relu_fwd_t(cudaStream_t s, const T* x, const T* r, T* out, const float* coef, size_t outer, int C)
+{
+	const size_t total = outer * C;
+	if (total == 0)
+		return 0;
+	constexpr int W = Vec16<T>::W;
+	const int CW = C / W;
+	if (C % W == 0 && (256 % CW == 0 || CW % 256 == 0) && aligned_v16(x) && aligned_v16(r) && aligned_v16(out))
+	{
+		// the launch rules of run_apply's channel-stationary path
+		int grid = grid_for(total / W / 4, 256);
+		if (CW > 256)
+			grid = (grid + CW / 256 - 1) / (CW / 256) * (CW / 256);
+		bn_apply_fixed_kernel<T, 0, 0, 0, 1><<<grid, 256, 0, s>>>(x, r, out, coef, total / W, C, 0);
+	} else
+		bn_apply_generic_kernel<T, 0, 0, 1><<<grid_for(total, 256), 256, 0, s>>>(x, r, out, coef, total, C, 1);
+	return check("bn_add_relu_fwd");
+}
+int bn_add_relu_fwd_f32(cudaStream_t s, const float* x, const float* r, float* out, const float* coef, size_t outer, int C) { return bn_add_relu_fwd_t<float>(s, x, r, out, coef, outer, C); }
+int bn_add_relu_fwd_16(cudaStream_t s, int kind, const void* x, const void* r, void* out, const float* coef, size_t outer, int C)
+{
+	return kind == 1 ? bn_add_relu_fwd_t<__nv_bfloat16>(s, (const __nv_bfloat16*)x, (const __nv_bfloat16*)r, (__nv_bfloat16*)out, coef, outer, C) : bn_add_relu_fwd_t<__half>(s, (const __half*)x, (const __half*)r, (__half*)out, coef, outer, C);
+}
+
+// Backward: g = y > 0 ? a + b : 0 (b may be NULL: y > 0 ? a : 0) stored to g, and in the same pass the partial rows of the
+// reduction the batch-norm backward behind it needs over (g, x), into part (room for part_cap rows of 2C floats).  The grid and
+// row walk are run_reduce's, so the rows are bit-identical to what bn_bwd_t would reduce from g itself.  *part_rows = the number
+// of rows written; 0 when the layout does not take the vector path (then only g is written, by the plain kernels).
+template <typename T>
+static int bn_add_relu_bwd_reduce_t(cudaStream_t s, const T* a, const T* b, const T* y, const T* x, const float* mean, T* g, size_t outer, int C, float* part, int part_cap, int* part_rows)
+{
+	*part_rows = 0;
+	const size_t n = outer * C;
+	if (n == 0)
+		return 0;
+	constexpr int W = Vec16<T>::W;
+	if (part && C % W == 0 && aligned_v16(x) && aligned_v16(g) && aligned_v16(a) && aligned_v16(y) && (!b || aligned_v16(b)))
+	{
+		int cpb;
+		dim3 grid;
+		reduce_config(outer, C / W, cpb, grid);
+		if ((int)grid.y <= part_cap)
+		{
+			bn_reduce_kernel<T, 2, 0><<<grid, 256, 0, s>>>(x, (const T*)0, mean, (const float*)0, outer, C, part, cpb, a, b, y, g);
+			*part_rows = (int)grid.y;
+			return check("bn_add_relu_bwd_reduce");
+		}
+	}
+	if (b)
+		return add_relu_bwd_t<T>(s, a, b, y, g, n);
+	if (ElemKind<T>::value == 0)
+		return ew_relu_bwd_f32(s, (const float*)a, (const float*)y, (float*)g, n);
+	return ew_relu_bwd_16(s, ElemKind<T>::value, a, y, g, n);
+}
+int bn_add_relu_bwd_reduce_f32(cudaStream_t s, const float* a, const float* b, const float* y, const float* x, const float* mean, float* g, size_t outer, int C, float* part, int part_cap, int* part_rows)
+{
+	return bn_add_relu_bwd_reduce_t<float>(s, a, b, y, x, mean, g, outer, C, part, part_cap, part_rows);
+}
+int bn_add_relu_bwd_reduce_16(cudaStream_t s, int kind, const void* a, const void* b, const void* y, const void* x, const float* mean, void* g, size_t outer, int C, float* part, int part_cap, int* part_rows)
+{
+	if (kind == 1)
+		return bn_add_relu_bwd_reduce_t<__nv_bfloat16>(s, (const __nv_bfloat16*)a, (const __nv_bfloat16*)b, (const __nv_bfloat16*)y, (const __nv_bfloat16*)x, mean, (__nv_bfloat16*)g, outer, C, part, part_cap, part_rows);
+	return bn_add_relu_bwd_reduce_t<__half>(s, (const __half*)a, (const __half*)b, (const __half*)y, (const __half*)x, mean, (__half*)g, outer, C, part, part_cap, part_rows);
 }
 
 } // namespace sm100

@@ -46,6 +46,12 @@ __device__ __forceinline__ void stf(float* p, const float v) { *p = v; }
 __device__ __forceinline__ void stf(__nv_bfloat16* p, const float v) { *p = __float2bfloat16_rn(v); }
 __device__ __forceinline__ void stf(__half* p, const float v) { *p = __float2half_rn(v); }
 
+// v rounded to the storage type T and back: what a store followed by a load of T gives (a no-op for fp32)
+template <typename T> __device__ __forceinline__ float rnd(const float v);
+template <> __device__ __forceinline__ float rnd<float>(const float v) { return v; }
+template <> __device__ __forceinline__ float rnd<__nv_bfloat16>(const float v) { return __bfloat162float(__float2bfloat16_rn(v)); }
+template <> __device__ __forceinline__ float rnd<__half>(const float v) { return __half2float(__float2half_rn(v)); }
+
 // element i of a buffer whose kind is only known at run time
 __device__ __forceinline__ float ld_kind(const void* p, const size_t i, const int kind)
 {

@@ -55,23 +55,33 @@ int pool_avg_bwd_16(cudaStream_t s, int kind, const PoolGeom& g, const void* gra
 // fuse_relu: y = relu(bn(x)) in the same pass (BATCH_NORM_FORWARD followed by an in-place RELU_FORWARD)
 // ext_part / ext_rows: per-channel statistics slots (four planes [ext_rows][C]: count, shift, shifted sum, shifted sum of squares) produced by the convolution that wrote x
 // (conv_stats_request); the statistics pass over x is then skipped
-int bn_fwd_train_f32(cudaStream_t s, const float* x, float* y, const float* scale, const float* bias, float* running_mean, float* running_var, float* saved_mean, float* saved_inv_std, size_t outer, int C, size_t inner, float epsilon, float momentum, void* workspace, int fuse_relu, const float* ext_part = 0, int ext_rows = 0);
+// coef_out: statistics only -- y is not written; the per-channel a, b of y = x * a + b go to coef_out[0, C) and [C, 2C)
+int bn_fwd_train_f32(cudaStream_t s, const float* x, float* y, const float* scale, const float* bias, float* running_mean, float* running_var, float* saved_mean, float* saved_inv_std, size_t outer, int C, size_t inner, float epsilon, float momentum, void* workspace, int fuse_relu, const float* ext_part = 0, int ext_rows = 0, float* coef_out = 0);
 size_t bn_workspace_bytes(int C);
 int bn_fwd_test_f32(cudaStream_t s, const float* x, float* y, const float* scale, const float* bias, const float* mean, const float* var, size_t outer, int C, size_t inner, float epsilon, void* workspace);
 // backward: dx, dscale, dbias from g, x, scale, saved_mean, saved_inv_std.  bias != NULL = fused with the RELU_BACKWARD
 // in front of it: g is masked by bn(x) > 0 on the fly (the mask is recomputed from x, bit-identical to the forward)
 // dx_colsum != NULL: also writes sum over rows of dx per channel (NHWC only; = the bias gradient of the convolution in front)
-int bn_bwd_f32(cudaStream_t s, const float* g, const float* x, const float* scale, const float* bias, const float* saved_mean, const float* saved_inv_std, float* dx, float* dscale, float* dbias, size_t outer, int C, size_t inner, void* workspace, float* dx_colsum = 0);
+// ext_part / ext_rows: the partial rows of the reduction over (g, x), already made by bn_add_relu_bwd_reduce_* (NHWC vector path only)
+int bn_bwd_f32(cudaStream_t s, const float* g, const float* x, const float* scale, const float* bias, const float* saved_mean, const float* saved_inv_std, float* dx, float* dscale, float* dbias, size_t outer, int C, size_t inner, void* workspace, float* dx_colsum = 0, const float* ext_part = 0, int ext_rows = 0);
 // the same on 16-bit activations (kind 1 = bf16, 2 = fp16): scale / bias / running and saved statistics / dscale / dbias stay fp32
 // (lib/nnc/ccv_cnnp_model_addons.c:954-956); dx_colsum is written in element kind colsum_kind (0 = fp32)
-int bn_fwd_train_16(cudaStream_t s, int kind, const void* x, void* y, const float* scale, const float* bias, float* running_mean, float* running_var, float* saved_mean, float* saved_inv_std, size_t outer, int C, size_t inner, float epsilon, float momentum, void* workspace, int fuse_relu, const float* ext_part = 0, int ext_rows = 0);
+int bn_fwd_train_16(cudaStream_t s, int kind, const void* x, void* y, const float* scale, const float* bias, float* running_mean, float* running_var, float* saved_mean, float* saved_inv_std, size_t outer, int C, size_t inner, float epsilon, float momentum, void* workspace, int fuse_relu, const float* ext_part = 0, int ext_rows = 0, float* coef_out = 0);
 int bn_fwd_test_16(cudaStream_t s, int kind, const void* x, void* y, const float* scale, const float* bias, const float* mean, const float* var, size_t outer, int C, size_t inner, float epsilon, void* workspace);
-int bn_bwd_16(cudaStream_t s, int kind, const void* g, const void* x, const float* scale, const float* bias, const float* saved_mean, const float* saved_inv_std, void* dx, float* dscale, float* dbias, size_t outer, int C, size_t inner, void* workspace, void* dx_colsum = 0, int colsum_kind = 0);
+int bn_bwd_16(cudaStream_t s, int kind, const void* g, const void* x, const float* scale, const float* bias, const float* saved_mean, const float* saved_inv_std, void* dx, float* dscale, float* dbias, size_t outer, int C, size_t inner, void* workspace, void* dx_colsum = 0, int colsum_kind = 0, const float* ext_part = 0, int ext_rows = 0);
 int ew_add_relu_fwd_16(cudaStream_t s, int kind, const void* a, const void* b, void* out, size_t n);
 int ew_add_relu_bwd_16(cudaStream_t s, int kind, const void* a, const void* b, const void* y, void* out, size_t n);
 // out = relu(a + b); out = y > 0 ? a + b : 0  (residual block end, forward / backward)
 int ew_add_relu_fwd_f32(cudaStream_t s, const float* a, const float* b, float* out, size_t n);
 int ew_add_relu_bwd_f32(cudaStream_t s, const float* a, const float* b, const float* y, float* out, size_t n);
+// residual block end with the batch norm of the main branch folded in (NHWC, C = innermost dimension):
+// forward  out = relu(roundT(x * coef[c] + coef[C + c]) + r), coef from bn_fwd_train_*(..., coef_out);
+// backward g = y > 0 ? a + b : 0 (b may be NULL) plus the partial rows of the batch-norm backward reduction over (g, x) in part
+//          (*part_rows of them, 0 when the layout takes the plain path), for bn_bwd_*(..., ext_part, ext_rows)
+int bn_add_relu_fwd_f32(cudaStream_t s, const float* x, const float* r, float* out, const float* coef, size_t outer, int C);
+int bn_add_relu_fwd_16(cudaStream_t s, int kind, const void* x, const void* r, void* out, const float* coef, size_t outer, int C);
+int bn_add_relu_bwd_reduce_f32(cudaStream_t s, const float* a, const float* b, const float* y, const float* x, const float* mean, float* g, size_t outer, int C, float* part, int part_cap, int* part_rows);
+int bn_add_relu_bwd_reduce_16(cudaStream_t s, int kind, const void* a, const void* b, const void* y, const void* x, const float* mean, void* g, size_t outer, int C, float* part, int part_cap, int* part_rows);
 
 // ---- softmax / losses over [batch, count] --------------------------------------------------------------------
 int softmax_fwd_f32(cudaStream_t s, const float* a, float* b, int batch, int count);
